@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W                (N>1: launched under torchrun, one rank/GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W   (the reference arm: CPU oracle port)
+  python bench.py ... --dump-outputs DIR                           (also writes the last timed step's outputs to DIR)
 
 A step = one pass of the hot path over one batch of synthetic frames.  `value` is whole-job FPS with
 frames resident in HBM; `e2e` is the same through the host-buffer C-ABI call (pinned H2D of the frames
@@ -22,6 +23,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # a benchmark run leaves the source tree as it found it (no __pycache__)
 
 METRIC = "detector FPS @1280x720 rpn300 (ResNet-101-FPN Faster-RCNN)"
 H, W, BATCH = 720, 1280, 8
@@ -219,6 +221,19 @@ def stream_record(cfg, device, precision, n_frames=48, opt_in=False):
             "timing": "host clock around synchronous calls (each call ends with a device sync)", "_dets": kept}
 
 
+def dump_outputs(det, out_dir):
+    """Writes the results the last timed pass left in the context -- what detect_device hands a caller that passes output
+    buffers -- as out_dir/<name>.npy: boxes [B,R,4], probs [B,R] and the box features [B*R,256,7,7] in float32, labels
+    [B,R] and valid [B] (detections per frame) as float64.  The frames and weights are seeded, so two builds run with the
+    same arguments can be compared array for array."""
+    os.makedirs(out_dir, exist_ok=True)
+    shapes = det.alloc_outputs(feat_mode=0)
+    for name, stage in (("boxes", "final_boxes"), ("probs", "final_probs"), ("labels", "final_labels"),
+                        ("valid", "final_count"), ("feat", "fpn_box_feat")):
+        a = det.get_stage(stage).reshape(shapes[name].shape)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+
+
 def reference_assoc_ms(dets_per_frame):
     """The reference's own association loop (deep_sort/tracker.py:57-138 restated in oracle/deepsort.py, numpy metric) on the
     detections the stream record fed to the native tracker: ms per frame on the host (part of cpu_baseline)."""
@@ -279,7 +294,13 @@ def main():
     ap.add_argument("--single-semantics", action="store_true", help="batch of 8 through the single-image graph semantics")
     ap.add_argument("--sustained-seconds", type=float, default=5.0, help="length of the sustained replay record (0 = skip)")
     ap.add_argument("--no-stream", action="store_true", help="skip the config-1 detect+track stream record")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0; about 40 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -334,6 +355,8 @@ def main():
     barrier()
     sampler.stop.set()
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(det, args.dump_outputs)     # before the records below run the context again
     # ---------------- sustained: the same graph replayed for >= 5 s (what the board settles at under its power cap) ----------------
     sustained = None
     if args.sustained_seconds > 0:

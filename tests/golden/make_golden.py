@@ -2,6 +2,7 @@
 (/root/reference: generate_anchors.py, deep_sort/*).  Run once in the authoring container:
     python tests/golden/make_golden.py
 The fixtures travel with the repo; /root/reference does not exist on the GPU box."""
+import hashlib
 import os
 import sys
 
@@ -178,8 +179,10 @@ def osnet():
     resized = np.stack([np.asarray(ext.to_pil(c).resize((128, 256), 2)) for c in crops])   # 2 = PIL BILINEAR
     d_cos = distance.compute_distance_matrix(torch.from_numpy(feats[:4]), torch.from_numpy(feats[2:]), "cosine").numpy()
     d_euc = distance.compute_distance_matrix(torch.from_numpy(feats[:4]), torch.from_numpy(feats[2:]), "euclidean").numpy()
+    # the crops are regenerated from the seed by the tests; their hashes pin that they are the same bytes
     np.savez_compressed(os.path.join(HERE, "osnet.npz"), feats=feats, resized=resized, d_cos=d_cos, d_euc=d_euc,
-                        **{"crop%d" % i: c for i, c in enumerate(crops)})
+                        crop_shapes=np.array([c.shape for c in crops], np.int64),
+                        crop_sha256=np.array([hashlib.sha256(c.tobytes()).hexdigest() for c in crops]))
 
 
 def effdet_numpy():

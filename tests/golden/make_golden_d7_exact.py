@@ -30,6 +30,6 @@ with frcnn.exact():
     r64 = oe.forward_from_features(cfg, Wt, {l: f64[l] for l in (3, 4, 5)}, image_scale=scale, stages=False)
 np.savez_compressed(os.path.join(HERE, "d7_exact.npz"), final_boxes=r64["final_boxes"], final_probs=r64["final_probs"],
                     final_labels=r64["final_labels"], levels=r64["levels"],
-                    c3=f64[3][:, ::8, ::8], c4=f64[4][:, ::4, ::4], c5=f64[5][:, ::2, ::2],     # strided samples of the endpoints
+                    c3=f64[3][:, ::8, ::8], c4=f64[4][:, ::4, ::4], c5=f64[5][:, ::4, ::4],     # strided samples of the endpoints
                     frame_checksum=np.int64(frame.astype(np.int64).sum()))
 print("written", os.path.join(HERE, "d7_exact.npz"))

@@ -96,6 +96,7 @@ def test_direct_epilogue_path_equals_tma_staged_epilogue():
     import os
     import subprocess
     import sys
+    import tempfile
     code = (
         "import numpy as np, sys; sys.path.insert(0, %r)\n"
         "from object_detection_tracking_b200 import engine\n"
@@ -107,10 +108,11 @@ def test_direct_epilogue_path_equals_tma_staged_epilogue():
         "o = engine.op_conv2d(x, w, b, r, pad=(1, 1, 1, 1), relu=True, split=True)\n"
         "np.save(sys.argv[1], o)\n") % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     outs = []
-    for i, env in enumerate([{}, {"B2_EPI_DIRECT": "1"}]):
-        path = "/tmp/b2_epi_%d.npy" % i
-        subprocess.run([sys.executable, "-c", code, path], check=True, env=dict(os.environ, **env), timeout=300)
-        outs.append(np.load(path))
+    with tempfile.TemporaryDirectory() as tmp:
+        for i, env in enumerate([{}, {"B2_EPI_DIRECT": "1"}]):
+            path = os.path.join(tmp, "epi_%d.npy" % i)
+            subprocess.run([sys.executable, "-c", code, path], check=True, env=dict(os.environ, **env), timeout=300)
+            outs.append(np.load(path))
     np.testing.assert_array_equal(outs[0], outs[1])
 
 

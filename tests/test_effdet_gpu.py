@@ -255,7 +255,7 @@ def test_d7_full_size_matches_oracle():
         gx = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "d7_exact.npz"))
         assert int(gx["frame_checksum"]) == int(frame.astype(np.int64).sum())
         ref64 = {k: gx[k] for k in ("final_boxes", "final_probs", "final_labels", "levels")}
-        strides = {3: 8, 4: 4, 5: 2}
+        strides = {3: 8, 4: 4, 5: 4}
         f64 = {l: gx["c%d" % l] for l in (3, 4, 5)}
         np.testing.assert_array_equal(eng.stage("image"), img)
         rec = {"config": "C3", "final": len(out["final_probs"]), "final_ref": len(ref["final_probs"])}

@@ -1,6 +1,7 @@
 """GPU parity of the two engines that build their own launch sequences on conv_tc_kernel beyond the detector: the vehicle
 ReID ResNet-101 (torchreid/models/resnet.py:441-455) against reference-generated activations (resnet101_reid.npz), and the
 Mask-RCNN head (--add_mask, models.py:934-961,1173-1199) against oracle.frcnn.maskrcnn_head.  First B200 run: round 2, 5/5 green."""
+import hashlib
 import os
 
 import numpy as np
@@ -12,6 +13,17 @@ pytestmark = pytest.mark.gpu
 @pytest.fixture(scope="module")
 def r101(golden_dir):
     return np.load(os.path.join(golden_dir, "resnet101_reid.npz"))
+
+
+def golden_crops(g):
+    """The ragged uint8 noise crops the fixture was generated from (seeded as in tests/golden/make_golden_tmot.py),
+    checked byte for byte against the hashes stored with it."""
+    rng = np.random.default_rng(15)
+    crops = [rng.integers(0, 256, (int(rng.integers(40, 200)), int(rng.integers(60, 320)), 3), dtype=np.uint8)
+             for _ in range(4)]
+    assert [c.shape for c in crops] == [tuple(s) for s in g["crop_shapes"]]
+    assert [hashlib.sha256(c.tobytes()).hexdigest() for c in crops] == list(g["crop_sha256"])
+    return crops
 
 
 def test_torch_style_strided_convs_single_op():
@@ -65,7 +77,7 @@ def test_resnet101_feature_extractor_drop_in(r101):
     from object_detection_tracking_b200.synth import synth_resnet101_reid_state
     ext = FeatureExtractor("resnet101", model_path="", image_size=(128, 256), device="cuda:0", batch=4,
                            state_dict=synth_resnet101_reid_state(2468))
-    crops = [r101["crop%d" % i] for i in range(4)]
+    crops = golden_crops(r101)
     got = ext(crops).numpy()
     assert got.shape == (4, 2048)
     assert np.abs(got - r101["feats"]).max() <= 3e-5 * np.abs(r101["feats"]).max()
