@@ -304,10 +304,11 @@ int b2_gallery_free(int device, float* dev);
 int b2_track_spatial_dist(const int32_t* frames1, const double* pts1, const int32_t* seg1, int N, const int32_t* frames2,
                           const double* pts2, const int32_t* seg2, int M, int frame_offset, double tol, double* out);
 
-/* Single-op entry used by the kernel parity tests (host pointers, NHWC activations, HWIO kernel). */
+/* Single-op entry used by the kernel parity tests (host pointers, NHWC activations, HWIO kernel).  a_mode: -1 automatic,
+ * 0 tiled 2-D A operand, 1 im2col; epi_mode: -1 automatic, 0 the direct per-thread epilogue. */
 int b2_op_conv2d(int device, const float* x, const float* w, const float* bias, const float* res, int B, int H, int W,
                  int Cin, int R, int S, int Cout, int stride, int dil, int pad_t, int pad_b, int pad_l, int pad_r,
-                 int relu, int res_shift, int impl, int split, int a_mode, float* out);
+                 int relu, int res_shift, int impl, int split, int a_mode, int epi_mode, float* out);
 
 /* Number of conv launches of this process that ran on CTA pairs (tcgen05 cta_group::2; opt-in through the environment
  * variable B2_PAIR=<min K-blocks>, DESIGN.md 4.3b): lets the tests assert that the hook is live. */

@@ -110,7 +110,7 @@ SYMBOLS = [
     ("b2_gallery_close", c_int, [c_int, c_void_p]),
     ("b2_gallery_free", c_int, [c_int, c_void_p]),
     ("b2_track_spatial_dist", c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, ctypes.c_double, c_void_p]),
-    ("b2_op_conv2d", c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p] + [c_int] * 18 + [c_void_p]),
+    ("b2_op_conv2d", c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p] + [c_int] * 19 + [c_void_p]),
     ("b2_conv_pair_launches", c_int64, []),
 ]
 

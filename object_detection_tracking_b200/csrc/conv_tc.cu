@@ -63,7 +63,6 @@ struct ConvTcParams {
   int acc_kb;        // ACC: K-blocks per tensor-core accumulation chunk
   int acc_ring;      // ACC: chunk accumulators in the TMEM ring (2 for 128-column tiles, 6 for 64-column tiles)
   int acc_stride;    // ACC: TMEM columns per accumulator (ring at 0.., the two correction accumulators after it)
-  int dbg_nodrain;   // perf experiment only (wrong results): skip the TMEM reads of the ACC drain
   float acc_delta;   // ACC: relative compensation of the tensor-core accumulator's truncation (kAccDelta)
   unsigned int* range_flag;   // ORed with 1 when a plane output exceeds the fp16 range (nullptr = not monitored)
   int epi_mode;      // 0 = direct global loads/stores per thread, 1 = TMA-staged (residual in, result out)
@@ -73,7 +72,6 @@ struct ConvTcParams {
   uint32_t epi_chunk_bytes;   // staged: bytes of one chunk buffer (4 KB hi plane, + 4 KB lo plane in split precision)
   uint32_t epi_off;  // byte offset of the epilogue staging buffers inside the tile area
   int num_pair_tiles;   // PAIR: tiles of 256 rows (two m-blocks, one per CTA of the pair) x block_n columns
-  int pair_bswap;       // PAIR, test hook: the CTAs load each other's half of the B tile
 };
 
 constexpr int kEpiSlotsMax = 3;
@@ -140,10 +138,8 @@ __device__ __forceinline__ void epilogue_chunk16(const ConvTcParams& p, float (&
     for (int j = 0; j < 4; ++j) o[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
     return;
   }
-#ifndef B2_NO_RANGE   // build variant for A/B runs: without the range monitor
 #pragma unroll
   for (int j = 0; j < 16; ++j) amax = fmaxf(amax, fabsf(v[j]));
-#endif
   uint32_t hi[8];
 #pragma unroll
   for (int j = 0; j < 8; ++j) hi[j] = pack_half2(v[2 * j], v[2 * j + 1]);
@@ -212,10 +208,8 @@ __device__ __forceinline__ void epilogue_chunk16_smem(const ConvTcParams& p, flo
 #pragma unroll
     for (int j = 0; j < 16; ++j) v[j] = __fmul_rn(v[j], 1.f / (1.f + expf(-v[j])));   // x * sigmoid(x) as the other kernels compute it
   }
-#ifndef B2_NO_RANGE   // build variant for A/B runs: without the range monitor
 #pragma unroll
   for (int j = 0; j < 16; ++j) amax = fmaxf(amax, fabsf(v[j]));
-#endif
   uint32_t hi[8];
 #pragma unroll
   for (int j = 0; j < 8; ++j) hi[j] = pack_half2(v[2 * j], v[2 * j + 1]);
@@ -399,14 +393,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
   __syncthreads();
   if (PAIR) cluster_sync();   // the peer's barriers are initialised before anything of this CTA signals them
   tc_fence_after();
-#ifdef B2_PDL
-  // Build variant (tools/build_variant.sh pdl -DB2_PDL=1), round-2 experiment: programmatic dependent launch.  The next
-  // conv of the stream may be scheduled onto SMs as they free up and run its prologue (barrier init, TMEM allocation,
-  // tensor-map prefetch -- everything above) while this grid is still in its last wave; it then waits here, before its
-  // first global-memory access, until the preceding grid has completed and flushed.
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
   const uint32_t tmem_base = *tmem_holder;
   if (tmem_base != 0) __trap();   // the MMA issuer addresses TMEM from column 0 / lane 0 (whole-TMEM allocation)
   // tile schedule: static round robin over CTAs (over CTA pairs in PAIR mode: pair tile = (m-block pair, n-block))
@@ -438,7 +424,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
         const int m_blk = PAIR ? 2 * m_row + static_cast<int>(crank) : m_row;   // an odd m-block count leaves the last
         const int m0 = m_blk * kBlockM;                                           // pair a block past M: TMA zero-fills it
         // PAIR: this CTA loads block_n/2 of the tile's B rows (the MMA reads the other half from the peer)
-        const int n0 = n_blk * p.block_n + (PAIR ? static_cast<int>(crank ^ static_cast<uint32_t>(p.pair_bswap)) * (p.block_n >> 1) : 0);
+        const int n0 = n_blk * p.block_n + (PAIR ? static_cast<int>(crank) * (p.block_n >> 1) : 0);
         int img = 0, ch = 0, cw = 0;
         if (p.a_mode == 1) {
           img = m0 / p.HoWo;
@@ -804,7 +790,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
             ecphase ^= 1;
           }
           tc_fence_after();
-          acc_fold<false, PAIR>(sums, tmem_base + lane_off + cbuf * p.acc_stride + c_beg * 16, p.dbg_nodrain ? 0 : my_n, &c_empty[cbuf], lane);
+          acc_fold<false, PAIR>(sums, tmem_base + lane_off + cbuf * p.acc_stride + c_beg * 16, my_n, &c_empty[cbuf], lane);
         }
         // the correction accumulator (hi*lo + lo*hi) is folded into the sums right away, which hands the tile's TMEM
         // stage back before the output stage starts
@@ -962,18 +948,6 @@ static int plan_build(ConvPlan* pl, const ConvDesc& d, const ConvWeights& w, con
   p.cin_blocks = d.Cin / kBlockK;
   p.num_kb = d.R * d.S * p.cin_blocks;
   p.block_n = pick_block_n(w.Cout_pad, split);
-  // short-K layers in split precision (K <= 256: at most four accumulation chunks per tile) are bound by the output
-  // stage; 64-column tiles leave TMEM room for a ring of six chunk accumulators, so the MMA issuer can run a whole tile
-  // ahead of the epilogue instead of stalling after two chunks (experiment hook until measured)
-  if (split && getenv("B2_SHORTK_BN64") != nullptr && p.num_kb <= 4 && p.block_n == 128 && w.Cout_pad % 64 == 0) p.block_n = 64;
-  // experiment hook (round 2): layers whose 128-column tiling ends in a nearly empty last wave (res4 at batch 8: 460
-  // tiles on 148 SMs = 3.1 waves, the 16 tiles of the 4th round cost a whole tile time) switch to 64-column tiles (920
-  // tiles = 6.2 waves of half the work: 3.5 instead of 4 tile times), at the price of twice the A-operand L2 traffic
-  if (split && getenv("B2_BN64_TAIL") != nullptr && p.block_n == 128 && w.Cout_pad % 64 == 0) {
-    const int tiles128 = ((d.B * Ho * Wo + kBlockM - 1) / kBlockM) * (w.Cout_pad / 128);
-    const int full = tiles128 / num_sms, rem = tiles128 % num_sms;
-    if (full >= 1 && full < 8 && rem > 0 && rem * 3 < num_sms) p.block_n = 64;
-  }
   p.num_n_blocks = w.Cout_pad / p.block_n;
   B2_CHECK(p.num_n_blocks * p.block_n == w.Cout_pad, "conv_tc: Cout_pad not divisible by block_n");
   const int num_m_blocks = (p.M + kBlockM - 1) / kBlockM;
@@ -984,12 +958,11 @@ static int plan_build(ConvPlan* pl, const ConvDesc& d, const ConvWeights& w, con
   pl->pair = false;
   if (const char* e = getenv("B2_PAIR")) {
     const int acc_kb_plan = d.acc_kb > 0 ? d.acc_kb : kAccChunkKb;
-    const bool acc_plan = split && d.acc_kb >= 0 && p.num_kb > acc_kb_plan && getenv("B2_NO_ACC") == nullptr;
+    const bool acc_plan = split && d.acc_kb >= 0 && p.num_kb > acc_kb_plan;
     pl->pair = acc_plan && atoi(e) > 0 && p.num_kb >= atoi(e) && p.block_n == 128 && d.relu != 2 && num_m_blocks >= 2 &&
                num_sms >= 2;
   }
   p.num_pair_tiles = ((num_m_blocks + 1) / 2) * p.num_n_blocks;
-  p.pair_bswap = getenv("B2_PAIR_BSWAP") != nullptr ? 1 : 0;
   p.idesc = make_idesc_f16(pl->pair ? 2 * kBlockM : kBlockM, p.block_n);
   p.b_bytes = static_cast<uint32_t>(pl->pair ? p.block_n / 2 : p.block_n) * kBlockK * 2;   // per CTA
   p.stage_bytes = (kABytes + p.b_bytes) * (split ? 2 : 1);
@@ -998,7 +971,6 @@ static int plan_build(ConvPlan* pl, const ConvDesc& d, const ConvWeights& w, con
     const bool one_to_one = d.off_h == 0 && d.off_w == 0 && d.out_H == Ho && d.out_W == Wo;
     const bool res_ok = io.res_hi == nullptr || (d.res_shift == 0 && d.res_H == d.out_H && d.res_W == d.out_W);
     p.epi_mode = (io.out_f32 == nullptr && one_to_one && res_ok && d.force_epi_mode != 0) ? 1 : 0;
-    if (getenv("B2_EPI_DIRECT") != nullptr) p.epi_mode = 0;   // test hook: exercise the per-thread epilogue
   }
   // staging rings (one per column half of the tile).  A group = epi_grp chunks of 16 columns that share one fence /
   // barrier / TMA-store round; a ring = epi_slots groups.  With a residual: three slots (the prefetch runs two groups
@@ -1015,11 +987,8 @@ static int plan_build(ConvPlan* pl, const ConvDesc& d, const ConvWeights& w, con
       return (kSmemBudget - epi) / static_cast<int>(p.stage_bytes);
     };
     if (p.epi_grp == 2 && stages_for(2) < (has_res ? 2 : 3) && stages_for(1) > stages_for(2)) p.epi_grp = 1;
-    if (const char* e = getenv("B2_EPI_GRP")) p.epi_grp = atoi(e) == 2 ? 2 : 1;   // experiment hooks
-    if (const char* e = getenv("B2_EPI_SLOTS_RES")) if (has_res) p.epi_slots = atoi(e) == 2 ? 2 : 3;
-    if (const char* e = getenv("B2_EPI_GRP_RES")) if (has_res) p.epi_grp = atoi(e) == 2 ? 2 : 1;
     // two-chunk groups move as one 32-column box per plane when every group of both halves is full
-    p.epi_wide = (p.epi_mode == 1 && p.epi_grp == 2 && nch % 4 == 0 && getenv("B2_EPI_NARROW") == nullptr) ? 1 : 0;
+    p.epi_wide = (p.epi_mode == 1 && p.epi_grp == 2 && nch % 4 == 0) ? 1 : 0;
     if (p.epi_mode != 1) {   // direct mode: no staging ring
       p.epi_grp = 1;
       p.epi_slots = 0;
@@ -1049,26 +1018,16 @@ static int plan_build(ConvPlan* pl, const ConvDesc& d, const ConvWeights& w, con
   p.res_shift = d.res_shift;
   p.relu = d.relu;
   pl->split = split;
-  // accurate accumulation: on by default in split precision when K spans more than one chunk
-  p.dbg_nodrain = getenv("B2_ACC_NODRAIN") != nullptr;
-  p.acc_delta = getenv("B2_ACC_DELTA") ? static_cast<float>(atof(getenv("B2_ACC_DELTA"))) : kAccDelta;
-  const float acc_delta2 = getenv("B2_ACC_DELTA2") ? static_cast<float>(atof(getenv("B2_ACC_DELTA2"))) : kAccDelta2;
   p.range_flag = io.range_flag;
+  // accurate accumulation: on by default in split precision when K spans more than one chunk
   p.acc_kb = d.acc_kb > 0 ? d.acc_kb : kAccChunkKb;
-  if (const char* e = getenv("B2_ACC_KB")) p.acc_kb = atoi(e) > 0 ? atoi(e) : kAccChunkKb;   // experiment hook
-  // experiment hook (round 2): two K-blocks per chunk on the K <= 256 layers only.  A 4-K-block tile then has two
-  // chunks = exactly the ring, so the MMA issuer can finish tile i+1 while the epilogue warps are still in the output
-  // stage of tile i (with one K-block per chunk it stalls after two of four), and the drains per tile halve; costs
-  // 8 instead of 4 truncating accumulation steps on those layers (all layers at 2: boxes 1.07e-3 px instead of 7.3e-4)
-  if (const char* e = getenv("B2_ACC_KB_SHORTK")) if (p.num_kb <= 4 && atoi(e) > 0) p.acc_kb = atoi(e);
   // experiment hook (round 2): longer chunks on the CTA-pair layers only -- every chunk hand-off of a pair crosses the two
   // SMs twice (commit multicast out, "drained" arrive back), which a two-deep ring of one-K-block chunks does not cover
   if (const char* e = getenv("B2_PAIR_ACC_KB")) if (pl->pair && atoi(e) > 0 && p.num_kb > atoi(e)) p.acc_kb = atoi(e);
-  pl->acc = split && d.acc_kb >= 0 && p.num_kb > p.acc_kb && getenv("B2_NO_ACC") == nullptr;
-  if (p.acc_kb >= 2) p.acc_delta = acc_delta2;
+  pl->acc = split && d.acc_kb >= 0 && p.num_kb > p.acc_kb;
+  p.acc_delta = p.acc_kb >= 2 ? kAccDelta2 : kAccDelta;
   p.acc_stride = p.block_n == 64 ? 64 : 128;
   p.acc_ring = p.block_n == 64 ? kAccRingMax : 2;   // (ring + 2 correction accumulators) * stride <= 512 columns
-  if (const char* e = getenv("B2_ACC_MIN_KB")) pl->acc = pl->acc && p.num_kb > atoi(e);   // experiment hook
   pl->grid = p.num_tiles < num_sms ? p.num_tiles : num_sms;
   if (pl->pair) {
     B2_CHECK(pl->acc && p.acc_ring == 2, "conv_tc: CTA pairs need the ACC scheme on 128-column tiles");
@@ -1160,37 +1119,11 @@ void conv_tc_plan_destroy(ConvPlan* p) { delete p; }
 static long long g_pair_launches = 0;   // launches that took the CTA-pair path (tests check that the opt-in hook is live)
 long long conv_tc_pair_launches() { return g_pair_launches; }
 
-#ifdef B2_PDL
-template <typename K>
-static cudaError_t launch_pdl(K kernel, const ConvPlan* pl, cudaStream_t stream) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(pl->grid);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = pl->smem_bytes;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, pl->tmA_hi, pl->tmA_lo, pl->tmB_hi, pl->tmB_lo, pl->tmO_hi, pl->tmO_lo, pl->tmR_hi,
-                            pl->tmR_lo, pl->p);
-}
-#endif
-
 int conv_tc_launch(const ConvPlan* pl, cudaStream_t stream) {
   const bool sw = pl->p.relu == 2;
 #define B2_CONV_LAUNCH(S, A, W)                                                                                          \
   conv_tc_kernel<S, A, W><<<pl->grid, kThreads, pl->smem_bytes, stream>>>(pl->tmA_hi, pl->tmA_lo, pl->tmB_hi, pl->tmB_lo, \
                                                                           pl->tmO_hi, pl->tmO_lo, pl->tmR_hi, pl->tmR_lo, pl->p)
-#ifdef B2_PDL
-  if (getenv("B2_PDL_OFF") == nullptr) {
-    if (pl->split && pl->acc) B2_CUDA(sw ? launch_pdl(conv_tc_kernel<true, true, true>, pl, stream) : launch_pdl(conv_tc_kernel<true, true, false>, pl, stream));
-    else if (pl->split) B2_CUDA(sw ? launch_pdl(conv_tc_kernel<true, false, true>, pl, stream) : launch_pdl(conv_tc_kernel<true, false, false>, pl, stream));
-    else B2_CUDA(sw ? launch_pdl(conv_tc_kernel<false, false, true>, pl, stream) : launch_pdl(conv_tc_kernel<false, false, false>, pl, stream));
-    return 0;
-  }
-#endif
   if (pl->pair) {
     ++g_pair_launches;
     cudaLaunchConfig_t cfg = {};

@@ -155,13 +155,8 @@ EConv* add_pw(b2_effdet* c, const std::string& wname, const std::string& biasnam
   // chunked re-accumulation (conv_tc ACC) on every layer with more than one K-block.  Round 1 switched it off up to
   // K = 512 for speed; at D7 depth (EfficientNet-b6: 45 blocks, then 8 BiFPN cells and 5-deep heads at 1536^2) the
   // truncation bias of up to 32 tensor-core accumulation steps per layer then compounds to 3e-5 relative on c5 -- six
-  // times the rounding noise of a float32 evaluation -- and boxes leave the 1e-3 px bar.  B2_EFFDET_ACC_MIN_K restores
-  // a threshold for throughput experiments.
-  {
-    static const int min_k = getenv("B2_EFFDET_ACC_MIN_K") ? atoi(getenv("B2_EFFDET_ACC_MIN_K")) : 0;
-    static const int chunk = getenv("B2_EFFDET_ACC_KB") ? atoi(getenv("B2_EFFDET_ACC_KB")) : 0;   // 0 = the kernel's default (1)
-    d.acc_kb = in.C <= min_k ? -1 : chunk;
-  }
+  // times the rounding noise of a float32 evaluation -- and boxes leave the 1e-3 px bar.
+  d.acc_kb = 0;   // the kernel's default chunk (one K-block)
   d.out_H = in.H; d.out_W = in.W; d.ldc = out_f32 ? ldc32 : out.C;
   L->w.Cout_pad = pad16(cout_real);
   L->w.K = in.C;
@@ -547,23 +542,19 @@ int launch_and_fetch(b2_effdet* c, bool full, float image_scale, float* boxes, f
                      float* box_feat, int* count) {
   B2_CUDA(cudaMemcpyAsync(c->scale_dev, &image_scale, 4, cudaMemcpyHostToDevice, c->stream));
   cudaGraphExec_t& graph = full ? c->graph_full : c->graph;
-  if (getenv("B2_EFFDET_NO_GRAPH") != nullptr) {
-    if (enqueue(c, full)) return -1;
-  } else {
-    if (!graph) {
-      if (enqueue(c, full)) return -1;           // eager warm-up before the capture
-      B2_CUDA(cudaStreamSynchronize(c->stream));
-      cudaGraph_t g = nullptr;
-      B2_CUDA(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-      const int rc = enqueue(c, full);
-      cudaError_t e = cudaStreamEndCapture(c->stream, &g);
-      if (rc) return -1;
-      B2_CUDA(e);
-      B2_CUDA(cudaGraphInstantiate(&graph, g, 0));
-      B2_CUDA(cudaGraphDestroy(g));
-    }
-    B2_CUDA(cudaGraphLaunch(graph, c->stream));
+  if (!graph) {
+    if (enqueue(c, full)) return -1;           // eager warm-up before the capture
+    B2_CUDA(cudaStreamSynchronize(c->stream));
+    cudaGraph_t g = nullptr;
+    B2_CUDA(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
+    const int rc = enqueue(c, full);
+    cudaError_t e = cudaStreamEndCapture(c->stream, &g);
+    if (rc) return -1;
+    B2_CUDA(e);
+    B2_CUDA(cudaGraphInstantiate(&graph, g, 0));
+    B2_CUDA(cudaGraphDestroy(g));
   }
+  B2_CUDA(cudaGraphLaunch(graph, c->stream));
   const int m = c->post.max_out;
   B2_CUDA(cudaMemcpyAsync(boxes, c->out_boxes, sizeof(float) * 4 * m, cudaMemcpyDeviceToHost, c->stream));
   B2_CUDA(cudaMemcpyAsync(scores, c->out_scores, sizeof(float) * m, cudaMemcpyDeviceToHost, c->stream));

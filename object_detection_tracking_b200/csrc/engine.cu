@@ -186,10 +186,9 @@ struct b2_ctx {
   cudaGraphExec_t graph = nullptr;
   // dual-stream pass: the backbone / FPN / RPN-head phases run as two half-batches on two streams, so that the tail of
   // one layer's persistent kernel (tiles % SMs != 0, no SM busy in the last round) overlaps the other half's kernels
-  bool dual = false;
-  int nsplit = 1;                                  // batch parts (= streams) of the forked phases
-  cudaStream_t side_stream[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  cudaEvent_t fork_ev = nullptr, join_ev[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  int nsplit = 1;                                  // batch parts (= streams) of the forked phases: 1 or 2
+  cudaStream_t side_stream = nullptr;
+  cudaEvent_t fork_ev = nullptr, join_ev = nullptr;
   bool weights_loaded = false;
   cudaEvent_t ev[NPHASE + 1];
   float phase_ms[NPHASE];
@@ -594,11 +593,8 @@ int build_plan(b2_ctx* c) {
     }
     // Images are independent through phases 0-2 (stem, ResNet, FPN, RPN head): a second set of plans covers each
     // half of the batch by itself (same tiles per image, so the results are bit-identical to the full-batch plan).
-    c->nsplit = 2;
-    if (const char* e = getenv("B2_SPLIT")) c->nsplit = atoi(e);   // experiment hook: 1, 2, 4, 8 batch parts
-    if (c->nsplit < 1 || c->nsplit > 8 || B % c->nsplit != 0) c->nsplit = 1;
-    c->dual = c->nsplit > 1 && getenv("B2_NO_DUAL") == nullptr;
-    if (c->dual) {
+    c->nsplit = B % 2 == 0 ? 2 : 1;
+    if (c->nsplit == 2) {
       for (const auto& s : c->steps) {
         if (s.kind != 0 || s.phase > 2) continue;
         Layer* L = s.layer;
@@ -722,23 +718,20 @@ int step_launches(const b2_ctx::Step& s) {
 // the capture through the fork event and rejoins before the proposals).
 int enqueue_dual(b2_ctx* c) {
   B2_CUDA(cudaEventRecord(c->fork_ev, c->stream));
-  for (int h = 1; h < c->nsplit; ++h) B2_CUDA(cudaStreamWaitEvent(c->side_stream[h - 1], c->fork_ev, 0));
+  B2_CUDA(cudaStreamWaitEvent(c->side_stream, c->fork_ev, 0));
   for (const auto& s : c->steps) {
     if (s.phase > 2) continue;
-    for (int h = 0; h < c->nsplit; ++h)
-      if (run_step_half(c, s, h, h == 0 ? c->stream : c->side_stream[h - 1])) return -1;
+    if (run_step_half(c, s, 0, c->stream) || run_step_half(c, s, 1, c->side_stream)) return -1;
   }
-  for (int h = 1; h < c->nsplit; ++h) {
-    B2_CUDA(cudaEventRecord(c->join_ev[h - 1], c->side_stream[h - 1]));
-    B2_CUDA(cudaStreamWaitEvent(c->stream, c->join_ev[h - 1], 0));
-  }
+  B2_CUDA(cudaEventRecord(c->join_ev, c->side_stream));
+  B2_CUDA(cudaStreamWaitEvent(c->stream, c->join_ev, 0));
   for (const auto& s : c->steps)
     if (s.phase > 2 && run_step(c, s)) return -1;
   return 0;
 }
 
 int enqueue(b2_ctx* c, int mask, bool with_events) {
-  if (c->dual && !with_events && mask == B2_PHASE_ALL) return enqueue_dual(c);
+  if (c->nsplit == 2 && !with_events && mask == B2_PHASE_ALL) return enqueue_dual(c);
   if (with_events) B2_CUDA(cudaEventRecord(c->ev[0], c->stream));
   int last = -1;
   for (const auto& s : c->steps) {
@@ -924,15 +917,13 @@ int b2_create(b2_ctx** out, int device, const b2_config* cfg) {
     b2_destroy(c.release());
     return -1;
   }
-  if (c->dual) {
+  if (c->nsplit == 2) {
     B2_CUDA(cudaEventCreateWithFlags(&c->fork_ev, cudaEventDisableTiming));
-    for (int h = 1; h < c->nsplit; ++h) {
-      B2_CUDA(cudaStreamCreateWithFlags(&c->side_stream[h - 1], cudaStreamNonBlocking));
-      B2_CUDA(cudaEventCreateWithFlags(&c->join_ev[h - 1], cudaEventDisableTiming));
-    }
+    B2_CUDA(cudaStreamCreateWithFlags(&c->side_stream, cudaStreamNonBlocking));
+    B2_CUDA(cudaEventCreateWithFlags(&c->join_ev, cudaEventDisableTiming));
   }
   c->launches = 0;
-  for (const auto& s : c->steps) c->launches += step_launches(s) * ((c->dual && s.phase <= 2) ? c->nsplit : 1);
+  for (const auto& s : c->steps) c->launches += step_launches(s) * (s.phase <= 2 ? c->nsplit : 1);
   B2_CUDA(cudaDeviceSynchronize());
   *out = c.release();
   return 0;
@@ -949,10 +940,8 @@ void b2_destroy(b2_ctx* c) {
       if (pp) conv_tc_plan_destroy(pp);
   }
   if (c->fork_ev) cudaEventDestroy(c->fork_ev);
-  for (int h = 0; h < 7; ++h) {
-    if (c->join_ev[h]) cudaEventDestroy(c->join_ev[h]);
-    if (c->side_stream[h]) cudaStreamDestroy(c->side_stream[h]);
-  }
+  if (c->join_ev) cudaEventDestroy(c->join_ev);
+  if (c->side_stream) cudaStreamDestroy(c->side_stream);
   if (c->raw_frames) cudaFree(c->raw_frames);
   if (c->h_range) cudaFreeHost(c->h_range);
   for (void* p : c->allocs) cudaFree(p);
@@ -1439,8 +1428,7 @@ int b2_set_stage(b2_ctx* c, const char* name, const void* src, int64_t bytes) {
 // one download on a private stream (round 1 allocated ~12 device buffers, encoded the tensor maps and freed everything
 // again on every call: 48 ms per JDE frame against 1.7 ms for numpy, profiles/r2_widen_timing_before_ws.jsonl).  Operands
 // are padded to the plan's shape with whatever the buffers hold (finite leftovers of earlier calls): padded rows / columns
-// only produce outputs nobody reads.  B2_NO_WS=1 (test hook) runs every call in a private workspace that is released
-// when the call returns -- same code, no reuse; tests compare the two bit for bit.
+// only produce outputs nobody reads.
 struct DistWs {
   int device = -1;
   cudaStream_t stream = nullptr;
@@ -1450,7 +1438,6 @@ struct DistWs {
   __half *a_hi = nullptr, *a_lo = nullptr, *b_hi = nullptr, *b_lo = nullptr;
   std::map<std::vector<int>, ConvPlan*> plans;   // key: Sp, Np, Dp, split
   int num_sms = 148;
-  bool transient = false;   // B2_NO_WS: owned by one call
   DistWs() = default;
   DistWs(const DistWs&) = delete;
   DistWs& operator=(const DistWs&) = delete;
@@ -1464,13 +1451,8 @@ struct DistWs {
     a_hi = a_lo = b_hi = b_lo = nullptr;
     cap_a = cap_b = cap_rows = cap_cols = cap_dp = 0;
   }
-  ~DistWs() {
-    if (!transient) return;   // the per-device workspaces live as long as the process (no CUDA calls at exit)
-    release();
-    if (stream) cudaStreamDestroy(stream);
-  }
 };
-static std::map<int, DistWs> g_dist_ws;
+static std::map<int, DistWs> g_dist_ws;   // lives as long as the process (no CUDA calls at exit)
 static std::map<int, int> g_num_sms;
 static std::mutex g_dist_ws_mutex;   // one call at a time per process (the trackers are single-threaded per stream)
 
@@ -1493,14 +1475,13 @@ static int dist_ws_reserve(DistWs& w, int device, int S, int N, int D, int Sp, i
     B2_CUDA(cudaStreamSynchronize(w.stream));
     const size_t o_a = w.cap_a, o_b = w.cap_b, o_r = w.cap_rows, o_c = w.cap_cols, o_d = w.cap_dp;
     w.release();                                          // the plans hold the old addresses
-    const size_t head = w.transient ? 1 : 2;              // only the dimension that overflowed grows (x2 head room)
-    auto grow = [head](size_t cap, size_t need, size_t floor_) {
-      return need > cap ? std::max(need * head, floor_) : std::max(cap, floor_);
+    auto grow = [](size_t cap, size_t need, size_t floor_) {   // only the dimension that overflowed grows (x2 head room)
+      return need > cap ? std::max(need * 2, floor_) : std::max(cap, floor_);
     };
     w.cap_a = grow(o_a, need_a, 1);
     w.cap_b = grow(o_b, need_b, 1);
-    w.cap_rows = grow(o_r, static_cast<size_t>(Sp), w.transient ? 128 : 256);
-    w.cap_cols = grow(o_c, static_cast<size_t>(Np), w.transient ? 16 : 256);
+    w.cap_rows = grow(o_r, static_cast<size_t>(Sp), 256);
+    w.cap_cols = grow(o_c, static_cast<size_t>(Np), 256);
     if (static_cast<size_t>(aux) > w.cap_rows + w.cap_cols) w.cap_rows = static_cast<size_t>(aux);
     w.cap_dp = std::max(o_d, static_cast<size_t>(Dp));
     B2_CUDA(cudaMalloc(&w.d_a, w.cap_a * 4));
@@ -1595,11 +1576,6 @@ int b2_cosine_cost(int device, const float* gallery, const int32_t* seg_offsets,
   B2_CUDA(cudaSetDevice(device));
   const bool split = precision == 1;
   std::lock_guard<std::mutex> lock(g_dist_ws_mutex);
-  if (getenv("B2_NO_WS") != nullptr) {
-    DistWs w;
-    w.transient = true;
-    return cosine_cost_run(w, device, gallery, seg_offsets, T, dets, N, D, split, cost);
-  }
   return cosine_cost_run(g_dist_ws[device], device, gallery, seg_offsets, T, dets, N, D, split, cost);
 }
 
@@ -1613,11 +1589,6 @@ int b2_distance_matrix(int device, const float* a, int na, const float* b, int n
   B2_CUDA(cudaSetDevice(device));
   const bool split = precision == 1;
   std::lock_guard<std::mutex> lock(g_dist_ws_mutex);
-  if (getenv("B2_NO_WS") != nullptr) {
-    DistWs w;
-    w.transient = true;
-    return distance_matrix_run(w, device, a, na, b, nb, D, metric, split, out);
-  }
   return distance_matrix_run(g_dist_ws[device], device, a, na, b, nb, D, metric, split, out);
 }
 
@@ -1626,14 +1597,14 @@ long long b2_conv_pair_launches(void) { return b2::conv_tc_pair_launches(); }
 
 int b2_op_conv2d(int device, const float* x, const float* w, const float* bias, const float* res, int B, int H, int W,
                  int Cin, int R, int S, int Cout, int stride, int dil, int pad_t, int pad_b, int pad_l, int pad_r,
-                 int relu, int res_shift, int impl, int split, int a_mode, float* out) {
+                 int relu, int res_shift, int impl, int split, int a_mode, int epi_mode, float* out) {
   B2_CHECK(x && w && out, "b2_op_conv2d: null argument");
   B2_CUDA(cudaSetDevice(device));
   ConvDesc d;
   d.B = B; d.in_H = H; d.in_W = W; d.Cin = Cin; d.in_pitch_H = H; d.in_pitch_W = W; d.in_ld = Cin;
   d.R = R; d.S = S; d.stride = stride; d.dil = dil;
   d.pad_t = pad_t; d.pad_b = pad_b; d.pad_l = pad_l; d.pad_r = pad_r;
-  d.Cout = Cout; d.relu = relu; d.force_a_mode = a_mode;
+  d.Cout = Cout; d.relu = relu; d.force_a_mode = a_mode; d.force_epi_mode = epi_mode;
   const int Ho = d.Ho(), Wo = d.Wo();
   B2_CHECK(Ho > 0 && Wo > 0, "b2_op_conv2d: empty output");
   const int Cp = (Cout + 15) / 16 * 16;

@@ -540,12 +540,6 @@ static int reid_embed_impl(b2_reid* c, const uint8_t* crops_host, int n, float* 
   const cudaMemcpyKind out_kind = to_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
   if (n < c->B) B2_CUDA(cudaMemsetAsync(c->crops + n * per, 0, (c->B - n) * per, c->stream));
   B2_CUDA(cudaMemcpyAsync(c->crops, crops_host, n * per, cudaMemcpyHostToDevice, c->stream));
-  if (getenv("B2_REID_NO_GRAPH") != nullptr) {
-    if (reid_enqueue(c)) return -1;
-    B2_CUDA(cudaMemcpyAsync(feats, c->feats, sizeof(float) * n * c->feat_dim, out_kind, c->stream));
-    B2_CUDA(cudaStreamSynchronize(c->stream));
-    return 0;
-  }
   if (!c->graph) {
     if (reid_enqueue(c)) return -1;                 // eager warm-up before the capture
     B2_CUDA(cudaStreamSynchronize(c->stream));

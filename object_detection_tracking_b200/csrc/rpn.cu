@@ -320,16 +320,14 @@ int rpn_proposals_launch(const RpnParams& p, cudaStream_t s) {
   }
   B2_CHECK(smem1 <= 200 * 1024 && smem2 <= 200 * 1024, "rpn: top-k too large for shared memory");
   {
-    // B2_RPN_CLUSTER=1 (test hook) runs the same kernel as single-CTA clusters
-    static const int cs = getenv("B2_RPN_CLUSTER") ? std::max(1, std::min(kRpnCluster, atoi(getenv("B2_RPN_CLUSTER")))) : kRpnCluster;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(5 * cs, p.B);
+    cfg.gridDim = dim3(5 * kRpnCluster, p.B);
     cfg.blockDim = dim3(1024);
     cfg.dynamicSmemBytes = smem1;
     cfg.stream = s;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = cs;
+    attr[0].val.clusterDim.x = kRpnCluster;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;

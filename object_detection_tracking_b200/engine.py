@@ -219,7 +219,7 @@ def cosine_cost(gallery: np.ndarray, seg_offsets: np.ndarray, dets: np.ndarray, 
 
 
 def op_conv2d(x, w, bias=None, res=None, stride=1, dil=1, pad=(0, 0, 0, 0), relu=False, res_shift=0,
-              impl="tcgen05", split=True, a_mode=-1, device=0) -> np.ndarray:
+              impl="tcgen05", split=True, a_mode=-1, epi_mode=-1, device=0) -> np.ndarray:
     """Single convolution through the C ABI (NHWC activations, HWIO kernel) -- used by the kernel tests."""
     lib = _lib.load()
     x = np.ascontiguousarray(x, dtype=np.float32)
@@ -234,7 +234,8 @@ def op_conv2d(x, w, bias=None, res=None, stride=1, dil=1, pad=(0, 0, 0, 0), relu
     r = None if res is None else np.ascontiguousarray(res, dtype=np.float32)
     _lib.check(lib.b2_op_conv2d(device, _lib.ptr(x), _lib.ptr(w), _lib.ptr(b), _lib.ptr(r), B, H, W, Cin, R, S, Cout,
                                 stride, dil, pt, pb, pl, pr, int(relu), int(res_shift),
-                                {"tcgen05": 0, "simt": 1}[impl], int(split), int(a_mode), _lib.ptr(out)),
+                                {"tcgen05": 0, "simt": 1}[impl], int(split), int(a_mode), int(epi_mode),
+                                _lib.ptr(out)),
                "b2_op_conv2d")
     return out
 

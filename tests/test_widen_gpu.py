@@ -246,9 +246,9 @@ def test_detect_then_track_loop_end_to_end():
 
 
 def test_distance_calls_from_the_persistent_workspace_equal_the_per_call_path():
-    """The default grow-only workspace + cached GEMM plans behind b2_cosine_cost / b2_distance_matrix returns the same bits as
-    a private workspace per call (B2_NO_WS=1), across growing and shrinking shapes and both metrics (each mode in its own process: the switch is
-    read from the environment)."""
+    """The default grow-only workspace + cached GEMM plans behind b2_cosine_cost / b2_distance_matrix returns the same bits,
+    across growing and shrinking shapes and both metrics, as each call made as the first call of a fresh process (a new
+    workspace sized for that call alone, with no leftovers of earlier calls)."""
     import subprocess
     import sys
     import tempfile
@@ -256,24 +256,32 @@ def test_distance_calls_from_the_persistent_workspace_equal_the_per_call_path():
         "import numpy as np, sys; sys.path.insert(0, %r)\n"
         "from object_detection_tracking_b200.engine import cosine_cost\n"
         "from object_detection_tracking_b200.reid import compute_distance_matrix\n"
+        "only = sys.argv[2] if len(sys.argv) > 2 else None   # run just this call\n"
         "rng = np.random.default_rng(0); out = {}\n"
         "for k, (T, per, N, D) in enumerate([(5, 3, 7, 64), (40, 5, 90, 256), (3, 2, 4, 256), (100, 5, 100, 256), (9, 4, 33, 48)]):\n"
         "    gal = np.abs(rng.standard_normal((T * per, D))).astype(np.float32) + 0.1\n"
         "    seg = (np.arange(T + 1) * per).astype(np.int32)\n"
         "    det = np.abs(rng.standard_normal((N, D))).astype(np.float32) + 0.1\n"
-        "    out['cos%%d' %% k] = cosine_cost(gal, seg, det)\n"
-        "    out['euc%%d' %% k] = compute_distance_matrix(gal, det, 'euclidean').numpy()\n"
-        "    out['cdm%%d' %% k] = compute_distance_matrix(det, gal, 'cosine').numpy()\n"
+        "    calls = {'cos%%d' %% k: lambda: cosine_cost(gal, seg, det),\n"
+        "             'euc%%d' %% k: lambda: compute_distance_matrix(gal, det, 'euclidean').numpy(),\n"
+        "             'cdm%%d' %% k: lambda: compute_distance_matrix(det, gal, 'cosine').numpy()}\n"
+        "    for name, call in calls.items():\n"
+        "        if only in (None, name):\n"
+        "            out[name] = call()\n"
         "np.savez(sys.argv[1], **out)\n") % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = []
+    names = ["%s%d" % (kind, k) for k in range(5) for kind in ("cos", "euc", "cdm")]
+    fresh = {}
     with tempfile.TemporaryDirectory() as tmp:
-        for i, env in enumerate([{"B2_NO_WS": "1"}, {}]):
-            path = os.path.join(tmp, "o%d.npz" % i)
-            subprocess.run([sys.executable, "-c", code, path], check=True, env=dict(os.environ, **env), timeout=300)
-            res.append(dict(np.load(path)))
-    assert set(res[0]) == set(res[1]) and len(res[0]) == 15
-    for k in res[0]:
-        np.testing.assert_array_equal(res[0][k], res[1][k])
+        path = os.path.join(tmp, "reused.npz")
+        subprocess.run([sys.executable, "-c", code, path], check=True, timeout=300)
+        reused = dict(np.load(path))
+        for name in names:
+            path = os.path.join(tmp, name + ".npz")
+            subprocess.run([sys.executable, "-c", code, path, name], check=True, timeout=300)
+            fresh.update(np.load(path))
+    assert set(reused) == set(fresh) == set(names)
+    for k in names:
+        np.testing.assert_array_equal(fresh[k], reused[k])
 
 
 def test_euclidean_nearest_neighbor_metric():

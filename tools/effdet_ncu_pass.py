@@ -1,5 +1,5 @@
-"""One eager EfficientDet pass bracketed by cudaProfilerStart/Stop, for ncu:
-  B2_EFFDET_NO_GRAPH=1 ncu --profile-from-start off --metrics gpu__time_duration.sum --clock-control none --csv \
+"""One EfficientDet pass bracketed by cudaProfilerStart/Stop, for ncu:
+  ncu --profile-from-start off --metrics gpu__time_duration.sum --clock-control none --csv \
       --log-file gpurun_out/effdet_launches.csv python tools/effdet_ncu_pass.py [det] [H] [W] [precision]
 A number printed under ncu is never a bench value."""
 import os
@@ -10,7 +10,6 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
-os.environ["B2_EFFDET_NO_GRAPH"] = "1"
 from gpu_effnet_probe import synth_frame  # noqa: E402
 from object_detection_tracking_b200.effdet import EffdetEngine  # noqa: E402
 from object_detection_tracking_b200.effdet_config import BACKBONE_OF, make_effdet_config  # noqa: E402

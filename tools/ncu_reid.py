@@ -1,4 +1,4 @@
-"""One eager OSNet-x1.0 embedding pass (batch 64) bracketed by cudaProfilerStart/Stop, for ncu (B2_REID_NO_GRAPH=1)."""
+"""One OSNet-x1.0 embedding pass (batch 64) bracketed by cudaProfilerStart/Stop, for ncu."""
 import os
 import sys
 
@@ -7,7 +7,6 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-os.environ["B2_REID_NO_GRAPH"] = "1"
 from object_detection_tracking_b200.reid import ReidEngine  # noqa: E402
 from object_detection_tracking_b200.synth import synth_osnet_state  # noqa: E402
 

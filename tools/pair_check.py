@@ -1,7 +1,7 @@
 """Bring-up check of the CTA-pair (cta_group::2) path of conv_tc_kernel: every eligible case of tests/test_conv_gpu.py and
 the res4 / FPN shapes of the detector, computed with B2_PAIR on and off in one process -- the two paths do the same
 arithmetic in the same order, so the outputs must be bit-identical.  On a mismatch prints which 128-row x 64-column blocks
-differ (a swapped B half or m-block shows as a pattern) and retries with B2_PAIR_BSWAP=1.
+differ (a swapped B half or m-block shows as a pattern).
 Usage: python tools/pair_check.py [min_kb]      exit code 0 = all identical"""
 import os
 import sys
@@ -20,19 +20,15 @@ EXTRA = {
 }
 
 
-def run(spec, x, w, bias, res, pair, bswap=False):
-    for k in ("B2_PAIR", "B2_PAIR_BSWAP"):
-        os.environ.pop(k, None)
+def run(spec, x, w, bias, res, pair):
+    os.environ.pop("B2_PAIR", None)
     if pair:
         os.environ["B2_PAIR"] = str(pair)
-    if bswap:
-        os.environ["B2_PAIR_BSWAP"] = "1"
     try:
         return engine.op_conv2d(x, w, bias, res, stride=spec[6], dil=spec[7], pad=spec[8], relu=bool(spec[10]),
                                 res_shift=spec[12], impl="tcgen05", split=True)
     finally:
         os.environ.pop("B2_PAIR", None)
-        os.environ.pop("B2_PAIR_BSWAP", None)
 
 
 def block_map(a, b):
@@ -69,8 +65,6 @@ def main():
             print("   blocks (rows of 128 down, columns of 64 across; first 12 rows): ")
             for ln in bm[:12]:
                 print("   " + ln)
-            sw = run(spec, x, w, bias, res, min_kb, bswap=True)
-            print("   with B2_PAIR_BSWAP=1: %s" % ("identical" if np.array_equal(base, sw) else "different"))
             d = np.abs(got.astype(np.float64) - base)
             print("   max |diff| %.3e at %s, finite %s" % (d.max(), np.unravel_index(d.argmax(), d.shape), np.isfinite(got).all()),
                   flush=True)
